@@ -9,7 +9,6 @@ for p in (ROOT, os.path.join(ROOT, "c-ray_b200"), os.path.join(ROOT, "tests")):
         sys.path.insert(0, p)
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-BUILT = os.path.join(ROOT, "scenes", "_built")
 GOLDEN_SCENES = ["g_nodes", "g_legacy", "g_single", "g_meshmat"]
 # + the fixture whose node graphs no JSON can express (SURVEY 8 f4: built by the reference's C constructors in oracle/ref_harness.c):
 # only its flat export exists, so the loader tests skip it
@@ -31,3 +30,37 @@ def _built():
     """Make sure the shared libraries exist (cheap no-op when they are already built)."""
     import __graft_entry__ as g
     g.build(quiet=True)
+
+
+@pytest.fixture(scope="session")
+def bundled_scene(tmp_path_factory):
+    """bundled_scene(name) -> path of the flat scene of the reference's bundled input/<name>.json (copied to oracle/_ref/input by
+    build()), made by this repository's loader (tests/test_loader.py holds it to the reference's own export), or None when
+    oracle/_ref/input is missing."""
+    import ctypes as C
+    import crgpu
+    import crscene
+    made = {}
+    refdir = os.path.join(ROOT, "oracle", "_ref")
+
+    def get(name):
+        if name not in made:
+            made[name] = None
+            if os.path.exists(os.path.join(refdir, "input", name + ".json")):
+                cwd = os.getcwd()
+                os.chdir(refdir)              # node-graph texture paths are relative to the reference's working directory
+                try:
+                    flat = crscene.load_json(os.path.join("input", name + ".json"))
+                finally:
+                    os.chdir(cwd)
+                path = str(tmp_path_factory.mktemp("bundled") / (name + ".crscene"))
+                L = crgpu.lib()
+                L.crscene_save.argtypes = [C.POINTER(crgpu.FlatScene), C.c_char_p]
+                assert L.crscene_save(C.byref(flat), path.encode()) == 0
+                crscene.free(flat)
+                made[name] = path
+        return made[name]
+    return get
+
+
+NO_BUNDLED = "oracle/_ref/input (the reference's bundled scenes, copied by build()) is missing"

@@ -95,21 +95,26 @@ def test_reference_main_program_on_the_b200_path(tmp_path, monkeypatch):
 
 
 @pytest.mark.gpu
-def test_reference_renderframe_with_the_gpu_worker_in_its_thread_slot(tmp_path):
+def test_reference_renderframe_with_the_gpu_worker_in_its_thread_slot(tmp_path, bundled_scene):
     """INTEGRATION.md §2, compiled and run: oracle/_ref/cray_ref_gpu is the UNMODIFIED reference (its loader, BVH builder, tile
     queue, renderFrame, stats loop) built by oracle/Makefile with the two integration files a maintainer adds
     (c-ray_b200/integration/gpu_thread.c + flatten_world.c) and libcrgpu.so.  With CRAY_GPU=1 renderFrame's thread-function slot
     (renderer.c:92-105) is filled with gpuRenderThread; the fp32 renderBuffer must match the CPU reference's."""
+    import oracle_lib as O
+    import reference_golden as RG
     exe = os.path.join(REF_DIR, "cray_ref_gpu")
-    ref_path = os.path.join(ROOT, "scenes", "_built", "ref_scene_320x200x16_b4.f32")
-    if not (os.path.exists(exe) and os.path.exists(ref_path)):
-        pytest.skip("oracle/_ref/cray_ref_gpu is built where /root/reference exists and travels with the repo")
+    scene = bundled_scene("scene")
+    if not (os.path.exists(exe) and scene):
+        pytest.skip("oracle/_ref/cray_ref_gpu and oracle/_ref/input are built by build() where the reference sources are present")
     out = str(tmp_path / "gpu.f32")
     r = subprocess.run([exe, "render", "input/scene.json", "320", "200", "16", "4", "1", "0", "0", out], cwd=REF_DIR,
                        env=dict(os.environ, CRAY_GPU="1"), stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=600)
     assert r.returncode == 0 and "REF_RENDER" in r.stdout, r.stdout[-2000:]
     got = np.fromfile(out, dtype=np.float32)
-    ref = np.fromfile(ref_path, dtype=np.float32)
+    o = O.OracleScene(scene, 320, 200, 16, 4)
+    ref = o.render(threads=os.cpu_count()).ravel()       # the strict reference's frame, bit for bit (checked by its digest)
+    o.close()
+    assert RG.frame_digest(ref) == RG.golden()["frames"][RG.frame_key("scene", 320, 200, 16, 4)]
     assert got.shape == ref.shape and np.isfinite(got).all()
     rmse = float(np.sqrt(((got.astype(np.float64) - ref) ** 2).mean()))
     assert rmse <= 1e-4, rmse
@@ -118,5 +123,4 @@ def test_reference_renderframe_with_the_gpu_worker_in_its_thread_slot(tmp_path):
     r = subprocess.run([exe, "render", "input/scene.json", "80", "50", "4", "4", "2", "0", "0", out2], cwd=REF_DIR,
                        env={k: v for k, v in os.environ.items() if k != "CRAY_GPU"}, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=600)
     assert r.returncode == 0
-    small = os.path.join(ROOT, "scenes", "_built", "ref_scene_80x50x4_b4.f32")
-    assert np.array_equal(np.fromfile(out2, dtype=np.float32).view(np.uint32), np.fromfile(small, dtype=np.float32).view(np.uint32))
+    assert RG.frame_digest(np.fromfile(out2, dtype=np.float32)) == RG.golden()["frames"][RG.frame_key("scene", 80, 50, 4, 4)]

@@ -11,7 +11,7 @@ import pytest
 
 import crgpu
 import crscene
-from conftest import GOLDEN, GOLDEN_SCENES, BUILT, ROOT
+from conftest import GOLDEN, GOLDEN_SCENES, NO_BUNDLED, ROOT
 
 
 def mesh_inputs(path):
@@ -107,12 +107,12 @@ def test_device_builder_equals_host_builder_on_synthetic_inputs():
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("scene", ["hdr", "scene", "refraction", "venus", "fence"])
-def test_device_builder_reproduces_the_bundled_scene_bvhs(scene):
-    """every mesh BVH of the bundled scenes (hdr.json: the 274,243-triangle Venus, 229,087 nodes) — stored there by the reference's
-    own loader (scenes/_built is exported by oracle/_ref) — rebuilt on the device: node for node, bit for bit."""
-    path = os.path.join(BUILT, scene + ".crscene")
-    if not os.path.exists(path):
-        pytest.skip("scenes/_built missing")
+def test_device_builder_reproduces_the_bundled_scene_bvhs(scene, bundled_scene):
+    """every mesh BVH of the bundled scenes (hdr.json: the 274,243-triangle Venus, 229,087 nodes) — as the host loader builds them,
+    the same as the reference's own loader (tests/test_loader.py) — rebuilt on the device: node for node, bit for bit."""
+    path = bundled_scene(scene)
+    if path is None:
+        pytest.skip(NO_BUNDLED)
     for label, bb, ct, nodes, prims in mesh_inputs(path):
         d_nodes, d_prims = crscene.build_bvh_gpu(bb, ct)
         same_tree(d_nodes, d_prims, nodes, prims)

@@ -11,7 +11,7 @@ import subprocess
 
 import pytest
 
-from conftest import ROOT, GOLDEN, GOLDEN_SCENES, GOLDEN_FLAT
+from conftest import ROOT, GOLDEN, GOLDEN_SCENES, GOLDEN_FLAT, NO_BUNDLED
 
 PKG = os.path.join(ROOT, "c-ray_b200")
 
@@ -48,10 +48,10 @@ def test_upload_bytes_do_not_depend_on_host_threads(harness, name):
     assert a[0] >= 13 * 256 and a == b == c
 
 
-def test_big_scene_threaded_repack_is_deterministic(harness):
-    scene = os.path.join(ROOT, "scenes", "_built", "hdr.crscene")
-    if not os.path.exists(scene):
-        pytest.skip("scenes/_built missing")
+def test_big_scene_threaded_repack_is_deterministic(harness, bundled_scene):
+    scene = bundled_scene("hdr")
+    if scene is None:
+        pytest.skip(NO_BUNDLED)
     a, b = uploads(harness, scene, 1), uploads(harness, scene, 8)
     assert a == b
     # PackedTri + ShadePoly + PairNode sections of hdr.json (274,245 triangles, 114,552 internal nodes) plus 23 MB of texels

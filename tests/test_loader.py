@@ -6,9 +6,10 @@ BVH node for node, same primitive order, same decoded textures — bit for bit, 
 the reference starts from identical inputs.
 
 Three layers:
-  * committed fixtures: tests/golden/*.json vs the *.crscene the strict reference exported (always run);
-  * the reference's bundled scenes (hdr, venus, refraction, scene) vs scenes/_built/*.crscene (when built here);
-  * differential fuzzing: random scenes written to a temp dir, loaded by both loaders (when oracle/_ref exists).
+  * committed fixtures: tests/golden/*.json vs the *.crscene the strict reference exported;
+  * the reference's bundled scenes (hdr, venus, refraction, scene, ...) vs digests of the reference's exports
+    (tests/golden/reference.json; the scenes themselves are copied to oracle/_ref/input by build());
+  * differential fuzzing: random scenes written to a temp dir vs digests of what the reference exported for them.
 Known, documented tolerances (reference reads uninitialised memory there): malloc slack in the global vertex buffer
 (slots past the parsed `v` lines), the unused bits of interior BVH nodes, and prefs.thread_count.
 """
@@ -18,17 +19,16 @@ import math
 import os
 import random
 import struct
-import subprocess
 import zlib
 
 import numpy as np
 import pytest
 
-from conftest import GOLDEN, BUILT, GOLDEN_SCENES, ROOT
+from conftest import GOLDEN, GOLDEN_SCENES, ROOT
 import crgpu
 import crscene
+import reference_golden as RG
 
-REF = os.path.join(ROOT, "oracle", "_ref", "cray_ref_strict")
 REF_INPUT = os.path.join(ROOT, "oracle", "_ref")
 
 
@@ -133,16 +133,13 @@ def test_golden_scene_matches_reference_export(name, monkeypatch):
     crscene.free(mine)
 
 
-@pytest.mark.parametrize("name", ["hdr", "venus", "refraction", "scene", "alphanode", "fence", "glowmetal", "statues", "uvsphere"])
+@pytest.mark.parametrize("name", RG.BUNDLED)
 def test_bundled_scene_matches_reference_export(name, monkeypatch):
-    src = os.path.join(REF_INPUT, "input", name + ".json")
-    exported = os.path.join(BUILT, name + ".crscene")
-    if not (os.path.exists(src) and os.path.exists(exported)):
-        pytest.skip("bundled scenes are copied/exported by build() only where /root/reference exists")
+    if not os.path.exists(os.path.join(REF_INPUT, "input", name + ".json")):
+        pytest.skip("oracle/_ref/input (the reference's bundled scenes, copied by build()) is missing")
     monkeypatch.chdir(REF_INPUT)
     mine = crscene.load_json(os.path.join("input", name + ".json"))
-    ref = load_crscene(exported)
-    assert_same_scene(mine, ref)
+    RG.assert_scene_matches(mine, RG.golden()["exports"]["bundled/" + name])
     crscene.free(mine)
 
 
@@ -464,23 +461,26 @@ def _fuzz_scene(rng, d):
             "display": {}, "camera": cam, "scene": {"ambientColor": amb, "primitives": prims, "meshes": meshes}}
 
 
-@pytest.mark.parametrize("seed", range(40))
-def test_fuzz_against_live_reference(seed, tmp_path, monkeypatch):
-    if not os.path.exists(REF):
-        pytest.skip("oracle/_ref/cray_ref_strict is only built where /root/reference exists")
+FUZZ_SEEDS = 40
+
+
+def write_fuzz_scene(seed, d):
+    """fuzz.json + its assets in d"""
     rng = random.Random(1000 + seed)
-    d = str(tmp_path)
     scene = _fuzz_scene(rng, d)
     if not scene["scene"]["primitives"] and not any(m["instances"] for m in scene["scene"]["meshes"]):
         scene["scene"]["primitives"] = [{"type": "sphere", "radius": 1, "instances": [{}], "color": [1, 0, 0], "bsdf": "metal"}]
     open(os.path.join(d, "fuzz.json"), "w").write(json.dumps(scene, indent=1))
+
+
+@pytest.mark.parametrize("seed", range(FUZZ_SEEDS))
+def test_fuzz_against_live_reference(seed, tmp_path, monkeypatch):
+    """random scenes against what the reference's loader exported for them (tests/reference_golden.py)"""
+    d = str(tmp_path)
+    write_fuzz_scene(seed, d)
     monkeypatch.chdir(d)
-    r = subprocess.run([REF, "export", "fuzz.json", "0", "0", "0", "0", "ref.crscene"], cwd=d, stdout=subprocess.PIPE,
-                       stderr=subprocess.STDOUT, text=True, timeout=120)
-    assert r.returncode == 0, r.stdout[-2000:]
     mine = crscene.load_json("fuzz.json")
-    ref = load_crscene(os.path.join(d, "ref.crscene"))
-    assert_same_scene(mine, ref)
+    RG.assert_scene_matches(mine, RG.golden()["exports"]["fuzz/%d" % seed])
     crscene.free(mine)
 
 
@@ -527,20 +527,13 @@ def test_large_mesh_same_for_any_thread_count(tmp_path, monkeypatch):
         A, B = crscene.arrays(scenes[0]), crscene.arrays(other)
         for key in A:
             assert A[key].tobytes() == B[key].tobytes(), key
-    if os.path.exists(REF):                                  # and the same as the reference's serial build
-        r = subprocess.run([REF, "export", "big.json", "0", "0", "0", "0", "ref.crscene"], cwd=d, stdout=subprocess.PIPE,
-                           stderr=subprocess.STDOUT, text=True, timeout=300)
-        assert r.returncode == 0, r.stdout[-2000:]
-        assert_same_scene(scenes[2], load_crscene(os.path.join(d, "ref.crscene")))
+    RG.assert_scene_matches(scenes[2], RG.golden()["exports"]["big"])      # and the same as the reference's serial build
     for s_ in scenes:
         crscene.free(s_)
 
 
-def test_texture_that_fails_late_falls_back_to_ordered_loading(tmp_path, monkeypatch):
-    """Textures are decoded on background threads; a file whose header is fine but whose deflate stream is corrupt is only
-    known to be bad after the node graph has been built with it.  The loader must then redo the load in order, ending with
-    the graph without an image node (a NULL texture makes no node, image.c:51) — same bytes with or without background decoding."""
-    d = str(tmp_path)
+def write_texture_fallback_scene(d):
+    """s.json with a good texture and one whose deflate stream is corrupt"""
     good = _png(5, 4, 2, 8, [bytes(range(15))] * 4)
     bad = bytearray(_png(64, 64, 6, 8, [bytes((x * 7 + y) & 255 for x in range(256)) for y in range(64)]))
     idat = bad.index(b"IDAT") + 4
@@ -551,6 +544,14 @@ def test_texture_that_fails_late_falls_back_to_ordered_loading(tmp_path, monkeyp
         {"type": "sphere", "radius": 1, "instances": [{}], "material": {"type": "diffuse", "color": {"type": "image", "path": "good.png"}}},
         {"type": "sphere", "radius": 1, "instances": [{}], "material": {"type": "metal", "color": {"type": "image", "path": "bad.png"}, "roughness": 0.3}}]}}
     open(os.path.join(d, "s.json"), "w").write(json.dumps(scene))
+
+
+def test_texture_that_fails_late_falls_back_to_ordered_loading(tmp_path, monkeypatch):
+    """Textures are decoded on background threads; a file whose header is fine but whose deflate stream is corrupt is only
+    known to be bad after the node graph has been built with it.  The loader must then redo the load in order, ending with
+    the graph without an image node (a NULL texture makes no node, image.c:51) — same bytes with or without background decoding."""
+    d = str(tmp_path)
+    write_texture_fallback_scene(d)
     monkeypatch.chdir(d)
     a = crscene.load_json("s.json")
     monkeypatch.setenv("CRLOADER_SYNC_TEXTURES", "1")
@@ -559,13 +560,11 @@ def test_texture_that_fails_late_falls_back_to_ordered_loading(tmp_path, monkeyp
     assert a.texture_count == 1 and a.node_count == b.node_count
     for key in A:
         assert A[key].tobytes() == B[key].tobytes(), key
-    if os.path.exists(REF):
-        r = subprocess.run([REF, "export", "s.json", "0", "0", "0", "0", "ref.crscene"], cwd=d, stdout=subprocess.PIPE,
-                           stderr=subprocess.STDOUT, text=True, errors="replace", timeout=60)
-        # the reference itself aborts on this input ("free(): invalid pointer": loadTextureFromBuffer destroys a texture that
-        # lives in the node pool, textureloader.c:78-84) — compare only if a build of it survives
-        if r.returncode == 0:
-            assert_same_scene(a, load_crscene(os.path.join(d, "ref.crscene")))
+    # the reference itself aborts on this input ("free(): invalid pointer": loadTextureFromBuffer destroys a texture that
+    # lives in the node pool, textureloader.c:78-84) — compare only if the build of it that made the golden data survived
+    ref = RG.golden()["exports"]["texture_fallback"]
+    if ref is not None:
+        RG.assert_scene_matches(a, ref)
     crscene.free(a); crscene.free(b)
 
 
@@ -625,27 +624,35 @@ def _odd_scene(rng, d):
     return sc
 
 
+ODD_SEEDS = 60
+
+
+def write_odd_scene(seed, d):
+    """s.json + its texture in d; False when the scene has a zero-sized image (the reference divides by zero there, the loader
+    reports it), so there is nothing to compare"""
+    rng = random.Random(777 + seed)
+    sc = _odd_scene(rng, d)
+    if any(k.lower() in ("width", "height") and v == 0 for k, v in sc.get("renderer", {}).items()):
+        return False
+    open(os.path.join(d, "s.json"), "w").write(json.dumps(sc))
+    return True
+
+
 def test_odd_inputs_against_live_reference(tmp_path, monkeypatch):
     """Defaults, clamps and fallbacks of the JSON dialect (sceneloader.c): 60 scenes made of values the loader has to
     tolerate — strings where numbers belong, missing radius/color/bsdf, lower-case keys, transforms without arguments,
-    mix/add nodes with missing inputs, unknown node and primitive types, textures that do not exist."""
-    if not os.path.exists(REF):
-        pytest.skip("oracle/_ref/cray_ref_strict is only built where /root/reference exists")
+    mix/add nodes with missing inputs, unknown node and primitive types, textures that do not exist — against what the
+    reference's loader exported for them (tests/reference_golden.py)."""
+    exports = RG.golden()["exports"]
     compared = 0
-    for seed in range(60):
-        rng = random.Random(777 + seed)
+    for seed in range(ODD_SEEDS):
         d = str(tmp_path / ("odd%d" % seed))
         os.makedirs(d)
-        sc = _odd_scene(rng, d)
-        if any(k.lower() in ("width", "height") and v == 0 for k, v in sc.get("renderer", {}).items()):
-            continue                                         # zero-sized image: the reference divides by zero, the loader reports it
-        open(os.path.join(d, "s.json"), "w").write(json.dumps(sc))
-        r = subprocess.run([REF, "export", "s.json", "0", "0", "0", "0", "ref.crscene"], cwd=d, stdout=subprocess.PIPE,
-                           stderr=subprocess.STDOUT, text=True, errors="replace", timeout=60)
-        assert r.returncode == 0, (seed, r.stdout[-500:])
+        if not write_odd_scene(seed, d):
+            continue
         monkeypatch.chdir(d)
         mine = crscene.load_json("s.json")
-        assert_same_scene(mine, load_crscene(os.path.join(d, "ref.crscene")))
+        RG.assert_scene_matches(mine, exports["odd/%d" % seed])
         crscene.free(mine)
         compared += 1
     assert compared >= 40

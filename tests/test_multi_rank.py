@@ -103,7 +103,7 @@ def test_gather_index_path_equals_tile_by_tile_copies():
         assert torch.equal(x, y)
 
 
-def test_rank_placement_balances_the_rays_of_the_headline_scene():
+def test_rank_placement_balances_the_rays_of_the_headline_scene(bundled_scene):
     """Static tile placement must spread the WORK, not just the tile count.  Dealing tiles by queue position (k % world) looks
     neutral but, under c-ray's default "fromMiddle" order, hands one rank every tile left of the image centre: on hdr.json the odd
     positions carry ~12% more rays (that was 0.88 instead of ~0.97 strong-scaling efficiency on 8 B200).  The spatial interleave of
@@ -112,10 +112,10 @@ def test_rank_placement_balances_the_rays_of_the_headline_scene():
     import pytest
     import crhost
     import oracle_lib as O
-    from conftest import BUILT
-    scene = os.path.join(BUILT, "hdr.crscene")
-    if not os.path.exists(scene):
-        pytest.skip("scenes/_built missing")
+    from conftest import NO_BUNDLED
+    scene = bundled_scene("hdr")
+    if scene is None:
+        pytest.skip(NO_BUNDLED)
     W, H, T = 480, 270, 16                                  # the 30 x 17 tile grid of 1920x1080 in 64x64 tiles
     R = crhost.Renderer(scene, W, H, 2, 32, gpus=1, tile=T, quiet=True)
     o = O.OracleScene(scene, W, H, 2, 32)
