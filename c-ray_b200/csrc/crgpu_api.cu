@@ -138,15 +138,13 @@ extern "C" void crgpu_host_free(void *p) { if (p) cudaFreeHost(p); }
  * crgpu_prepare() does everything about a scene that does not depend on the device: validation, BVH re-layout into pair nodes,
  * triangle packing, shading records.  crgpu_scene_create_prepared() is then one host->device copy of the slab plus two small
  * pointer-carrying tables.  A host that renders many frames of one scene, or one frame on many GPUs, prepares once. */
-enum { SEC_STAGE, SEC_PAIRS, SEC_TRIS, SEC_SLOT_POLY, SEC_SPOLYS, SEC_TOP_PRIMS, SEC_BVHS, SEC_INSTS, SEC_MATS, SEC_NODES, SEC_TEXS, SEC_LUT, SEC_TEXDATA, SEC_COUNT };
+enum { SEC_PAIRS, SEC_TRIS, SEC_SLOT_POLY, SEC_SPOLYS, SEC_TOP_PRIMS, SEC_BVHS, SEC_INSTS, SEC_MATS, SEC_NODES, SEC_TEXS, SEC_LUT, SEC_TEXDATA, SEC_COUNT };
 struct crgpu_prepared {
 	crs_prefs prefs;
 	crs_camera camera;
 	int32_t background;
 	uint32_t instance_count;
 	DevBvh top;
-	float world_lo[3], world_inv[3];
-	uint32_t stage_pairs;
 	uint32_t texture_count;
 	bool xnodes;               /* some node is of a kind only the complete interpreter (NodeX) evaluates */
 	uint8_t *slab;
@@ -415,7 +413,7 @@ static int alloc_wave(crgpu_scene *s, uint64_t paths, int sets) {
 	}
 	s->wave = nullptr; s->wave_bytes = 0; s->cap_paths = 0; s->wave_sets = 0;
 	const size_t n = ((size_t)paths + 255u) & ~(size_t)255u;      /* every sub-array stays 256-byte aligned */
-	const size_t per_set = n * (9u * 16u + 2u * 4u + 1u);         /* 153 B per path */
+	const size_t per_set = n * (8u * 16u + 2u * 4u + 1u);         /* 137 B per path */
 	const size_t bytes = per_set * (size_t)sets;
 	void *base = nullptr;
 	int rc = ctx_alloc(s->device, bytes, &base);
@@ -431,7 +429,6 @@ static int alloc_wave(crgpu_scene *s, uint64_t paths, int sets) {
 		w.hit = (float4 *)take(n * 16); w.L = (float4 *)take(n * 16);
 		w.hitInst = (int *)take(n * 4); w.perm = (unsigned *)take(n * 4);
 		w.hitKey = (unsigned char *)take(n);
-		w.perm2 = (unsigned *)take(n * 4); w.dirKey = (unsigned char *)take(n);
 	}
 	s->cap_paths = paths;
 	s->wave_sets = sets;
@@ -688,54 +685,14 @@ extern "C" int crgpu_prepare(const struct crs_scene *f, crgpu_prepared **out) {
 
 	std::vector<crs_node> nodes(f->nodes, f->nodes + f->node_count);
 
-	/* staging image: top-of-tree pair nodes (BFS prefix) of every BVH, the top level first, then the meshes
-	 * in proportion to their size, CRG_STAGE_PAIRS nodes in total */
-	std::vector<PairNode> stage;
-	{
-		auto take = [&](DevBvh &b, uint32_t quota) {
-			const uint32_t internal = b.node_count > 1 ? (uint32_t)(b.pair_end - b.pair_offset) : 0u;
-			const uint32_t cnt = quota < internal ? quota : internal;
-			b.stage_base = (uint32_t)stage.size();
-			b.stage_count = cnt;
-			stage.insert(stage.end(), pairs.begin() + b.pair_offset, pairs.begin() + b.pair_offset + cnt);
-		};
-		/* shared memory and L1 share 228 KB per SM: every staged KB is a KB of L1 the traversal loses, so the default
-		 * stages only the very top (128 nodes = 8 KB); CRGPU_TRACE_STAGE=<pairs> (0..1024) overrides */
-		const char *env = getenv("CRGPU_TRACE_STAGE");
-		uint32_t total_budget = env ? (uint32_t)atoi(env) : 0u;
-		if (total_budget > CRG_STAGE_PAIRS) total_budget = CRG_STAGE_PAIRS;
-		take(bvhs[f->top_bvh], total_budget / 4);
-		uint64_t total_internal = 0;
-		for (uint32_t b = 0; b < f->bvh_count; ++b) if (b != f->top_bvh && bvhs[b].node_count > 1) total_internal += bvhs[b].pair_end - bvhs[b].pair_offset;
-		const uint32_t budget = total_budget > (uint32_t)stage.size() ? total_budget - (uint32_t)stage.size() : 0u;
-		for (uint32_t b = 0; b < f->bvh_count && total_internal; ++b) {
-			if (b == f->top_bvh) continue;
-			const uint64_t internal = bvhs[b].node_count > 1 ? bvhs[b].pair_end - bvhs[b].pair_offset : 0;
-			take(bvhs[b], (uint32_t)((uint64_t)budget * internal / total_internal));
-		}
-	}
 	p->top = bvhs[f->top_bvh];
-	p->stage_pairs = (uint32_t)stage.size();
-	{	/* world bounds = bounds of the top-level BVH root (both children of pair 0, or the single leaf's box) */
-		float lo[3] = { 0.f, 0.f, 0.f }, hi[3] = { 1.f, 1.f, 1.f };
-		const crs_bvh &tb = f->bvhs[f->top_bvh];
-		if (tb.node_count >= 1) {
-			const float *b = f->bvh_nodes[tb.node_offset].bounds;          /* minx,maxx,miny,maxy,minz,maxz */
-			for (int k = 0; k < 3; ++k) { lo[k] = b[2 * k]; hi[k] = b[2 * k + 1]; }
-		}
-		for (int k = 0; k < 3; ++k) {
-			const float e = hi[k] - lo[k];
-			p->world_lo[k] = lo[k];
-			p->world_inv[k] = (e > 0.f && e < 3.0e38f) ? 1.0f / e : 0.f;
-		}
-	}
 	std::vector<float> lut(256);
 	for (int i = 0; i < 256; ++i) { volatile float num = (float)i, den = 255.0f; lut[i] = num / den; }   /* IEEE divss == __fdiv_rn */
 
 	/* lay the sections out in one slab (256-byte aligned each) and copy them in on the host threads */
-	const void *src[SEC_COUNT] = { stage.data(), pairs.data(), tris.data(), slot_poly.data(), spolys.data(), top_prims.data(), bvhs.data(),
+	const void *src[SEC_COUNT] = { pairs.data(), tris.data(), slot_poly.data(), spolys.data(), top_prims.data(), bvhs.data(),
 								   insts.data(), mats.data(), nodes.data(), texs.data(), lut.data(), f->texdata };
-	const size_t len[SEC_COUNT] = { stage.size() * sizeof(PairNode), pairs.size() * sizeof(PairNode), tris.size() * sizeof(PackedTri),
+	const size_t len[SEC_COUNT] = { pairs.size() * sizeof(PairNode), tris.size() * sizeof(PackedTri),
 									slot_poly.size() * sizeof(uint32_t), spolys.size() * sizeof(ShadePoly), top_prims.size() * sizeof(int32_t),
 									bvhs.size() * sizeof(DevBvh), insts.size() * sizeof(DevInstance), mats.size() * sizeof(DevMaterial),
 									nodes.size() * sizeof(crs_node), texs.size() * sizeof(DevTexture), lut.size() * sizeof(float), (size_t)f->texdata_bytes };
@@ -818,9 +775,6 @@ extern "C" int crgpu_scene_create_prepared(const crgpu_prepared *p, int device, 
 	d.background = p->background;
 	d.instance_count = p->instance_count;
 	d.top = p->top;
-	d.stage_pairs = p->stage_pairs;
-	memcpy(d.world_lo, p->world_lo, sizeof d.world_lo); memcpy(d.world_inv, p->world_inv, sizeof d.world_inv);
-	d.stage_img = reinterpret_cast<const PairNode *>(base + p->off[SEC_STAGE]);
 	d.pairs = reinterpret_cast<const PairNode *>(base + p->off[SEC_PAIRS]);
 	d.tris = reinterpret_cast<const PackedTri *>(base + p->off[SEC_TRIS]);
 	d.slot_poly = reinterpret_cast<const uint32_t *>(base + p->off[SEC_SLOT_POLY]);
@@ -839,26 +793,26 @@ extern "C" int crgpu_scene_create_prepared(const crgpu_prepared *p, int device, 
 	s->fb_floats = (size_t)d.image_width * d.image_height * 3u;
 	{ void *q = nullptr; FAIL_IF(ctx_alloc(device, s->fb_floats * sizeof(float), &q)); s->fb = static_cast<float *>(q); }
 	CUS(cudaMemsetAsync(s->fb, 0, s->fb_floats * sizeof(float), s->stream));
-	{	/* per wave set: hist[1024] + counts[64]; then the shared stats[80] */
-		const size_t set_bytes = 1024 * sizeof(unsigned) + 256;
+	{	/* per wave set: hist[512] + counts[64]; then the shared stats[80] */
+		const size_t set_bytes = 512 * sizeof(unsigned) + 256;
 		s->small_bytes = 2 * set_bytes + 80 * sizeof(unsigned long long);
 		FAIL_IF(ctx_alloc(device, s->small_bytes, &s->small));
 		CUS(cudaMemsetAsync(s->small, 0, s->small_bytes, s->stream));
 		uint8_t *sm = static_cast<uint8_t *>(s->small);
 		s->wb.hist = reinterpret_cast<unsigned *>(sm);
-		s->wb.counts = s->wb.hist + 1024;
+		s->wb.counts = s->wb.hist + 512;
 		s->wb2.hist = reinterpret_cast<unsigned *>(sm + set_bytes);
-		s->wb2.counts = s->wb2.hist + 1024;
+		s->wb2.counts = s->wb2.hist + 512;
 		s->wb.stats = s->wb2.stats = reinterpret_cast<unsigned long long *>(sm + 2 * set_bytes);
 	}
 	{
 		/* Paths in flight per wavefront batch.  Every batch pays a fixed ~7 ms (the serial chain of its bounces: each
 		 * late bounce lasts as long as its slowest ray), so batches should be as large as memory allows:
-		 * 153 B of wavefront state per path; use at most 40% of the free HBM (cached blocks count as free), capped at 256M paths. */
+		 * 137 B of wavefront state per path; use at most 40% of the free HBM (cached blocks count as free), capped at 256M paths. */
 		size_t free_b = 0, total_b = 0;
 		CUS(cudaMemGetInfo(&free_b, &total_b));
 		free_b += ctx_cached_bytes(device);
-		uint64_t fit = (uint64_t)((double)free_b * 0.40 / 153.0);
+		uint64_t fit = (uint64_t)((double)free_b * 0.40 / 137.0);
 		if (fit > (256ull << 20)) fit = 256ull << 20;
 		if (fit < (1ull << 20)) fit = 1ull << 20;
 		s->max_paths = fit;
@@ -939,12 +893,11 @@ static int render_pixels(crgpu_scene *s, TileDesc base, uint64_t tile_pixels, in
 	 * as long as its slowest ray.  So (1) batches are as large as the path budget allows and of EQUAL size (a 987 + 13 split wastes
 	 * a whole tail on 13 passes), and (2) with two or more batches the budget is split into two wave sets that run on two streams:
 	 * the thin tail of one batch overlaps the fat first bounces of the next.  Only the accumulate step is ordered (the running
-	 * average is taken in pass order, renderer.c:288-291): batch b's k_accumulate waits for batch b-1's.  CRGPU_OVERLAP=0 disables. */
-	static const int overlap_on = [] { const char *e = getenv("CRGPU_OVERLAP"); return e ? atoi(e) : 1; }();
+	 * average is taken in pass order, renderer.c:288-291): batch b's k_accumulate waits for batch b-1's. */
 	uint64_t batch = s->max_paths / tile_pixels;
 	if (batch < 1) batch = 1;
 	int sets = 1;
-	if (overlap_on && !timing && !count && batch < (uint64_t)pass_count && batch >= 2) { sets = 2; batch /= 2; }
+	if (!timing && !count && batch < (uint64_t)pass_count && batch >= 2) { sets = 2; batch /= 2; }
 	if (batch > (uint64_t)pass_count) batch = (uint64_t)pass_count;
 	{
 		const uint64_t nb = ((uint64_t)pass_count + batch - 1) / batch;
@@ -956,7 +909,6 @@ static int render_pixels(crgpu_scene *s, TileDesc base, uint64_t tile_pixels, in
 
 	const int maxDepth = (int)s->dev.bounces;
 	const int grid = s->sm_count * 8;
-	const int dirmode = crg_dir_mode();
 	uint64_t launches = 0;
 	float trace_ms = 0.f, shade_ms = 0.f;
 	if (timing) CU(cudaEventRecord(s->ev[0], s->stream));
@@ -982,14 +934,12 @@ static int render_pixels(crgpu_scene *s, TileDesc base, uint64_t tile_pixels, in
 		for (int depth = 0; depth < maxDepth; ++depth) {
 			if (depth >= CRG_TAIL_FROM && !count) { crg_launch_tail(s->dev_copy, wb, cur, depth, maxDepth, s->xnodes, st); ++launches; }
 			if (timing) { cudaEvent_t e; cudaEventCreate(&e); cudaEventRecord(e, st); tev.push_back(e); }
-			crg_launch_trace(s->dev, wb, cur, count, dirmode != 0 && depth > 0, grid, st);
+			crg_launch_trace(s->dev, wb, cur, count, st);
 			if (timing) { cudaEvent_t e; cudaEventCreate(&e); cudaEventRecord(e, st); tev.push_back(e); }
 			crg_launch_bucket(wb, cur, grid, st);
-			const bool sort_next = dirmode != 0 && depth + 1 < maxDepth;
-			crg_launch_shade(s->dev_copy, wb, cur, depth, maxDepth, sort_next ? dirmode : 0, s->xnodes, grid, st);
-			if (sort_next) { crg_launch_dirsort(wb, cur ^ 1, grid, st); ++launches; }    /* K4b: the next bounce's rays by direction bin */
+			crg_launch_shade(s->dev_copy, wb, cur, depth, maxDepth, s->xnodes, grid, st);
 			if (timing) { cudaEvent_t e; cudaEventCreate(&e); cudaEventRecord(e, st); tev.push_back(e); }
-			launches += 2 + (uint64_t)crg_shade_launches_per_bounce();
+			launches += 4;                                                       /* K2, K4, K3 miss half, K3 hit half */
 			cur ^= 1;
 		}
 		if (sets == 2 && bi > 0) CU(cudaStreamWaitEvent(st, s->evAcc[set ^ 1], 0));      /* pass order of the running average */
@@ -1014,8 +964,6 @@ static int render_pixels(crgpu_scene *s, TileDesc base, uint64_t tile_pixels, in
 			cudaEventElapsedTime(&a, tev[i], tev[i + 1]);
 			cudaEventElapsedTime(&b, tev[i + 1], tev[i + 2]);
 			trace_ms += a; shade_ms += b;
-			if (getenv("CRGPU_DUMP_TIMES") && (a > 5.f || b > 8.f || atoi(getenv("CRGPU_DUMP_TIMES")) > 1))
-				fprintf(stderr, "crgpu: batch %zu depth %zu trace %.3f ms shade %.3f ms\n", (i / 3) / (size_t)maxDepth, (i / 3) % (size_t)maxDepth, a, b);
 		}
 		for (cudaEvent_t e : tev) cudaEventDestroy(e);
 		s->pend_trace_ms += trace_ms; s->pend_shade_ms += shade_ms; s->pend_total_ms += total_ms;

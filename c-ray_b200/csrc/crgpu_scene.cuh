@@ -8,8 +8,7 @@
  *   PairNode  64 B, 64-B aligned: BOTH children of one internal node (bounds + refs), because the
  *             traversal always fetches and tests the two children together (bvh.c:392-398).  One
  *             LDG.128 x4 per step instead of two dependent 32-B fetches; internal nodes are renumbered
- *             in BFS order so the top of each tree is one contiguous range (staged into shared memory
- *             by TMA bulk copies in the traversal kernel).
+ *             in BFS order, so the top of each tree is one contiguous range.
  *   PackedTri 48 B, 16-B aligned, in LEAF ORDER (indexed by primIndices slot, not by poly): v0, e1, e2
  *             and n = e1 x e2 precomputed with the reference's exact fp32 operations (poly.c:20-22), so
  *             a leaf's triangles are contiguous and the Möller–Trumbore test needs no index chasing.
@@ -26,7 +25,6 @@
 
 #define CRG_LEAF_BIT 0x80000000u
 #define CRG_MAX_STACK 64            /* MAX_BVH_DEPTH, bvh.c:32 */
-#define CRG_STAGE_PAIRS 1024         /* 64 KB of shared memory per block for the staged top-of-tree nodes */
 
 struct __align__(64) PairNode {
 	float lb[6];                    /* left child: minx,maxx,miny,maxy,minz,maxz */
@@ -54,8 +52,6 @@ struct DevBvh {
 	uint32_t slot_offset;           /* into tris[] / slot_poly[] (mesh) or top_prims[] (top level) */
 	uint32_t root_first, root_count;/* when node_count == 1: the root is a leaf */
 	float    root_bounds[6];
-	uint32_t stage_base;            /* the first stage_count pair nodes (BFS order = top of the tree) of this BVH are also */
-	uint32_t stage_count;           /* in the staging image at [stage_base, stage_base+stage_count) — see DevScene.stage_img */
 	uint32_t pad;
 };
 
@@ -109,9 +105,5 @@ struct DevScene {
 	const DevMaterial*materials;
 	const crs_node   *nodes;
 	const DevTexture *textures;
-	const PairNode   *stage_img;    /* top-of-tree pair nodes of every BVH, contiguous: K2 copies it into shared memory with one
-	                                   TMA bulk copy (cp.async.bulk) per block; stage_pairs = number of nodes in it */
-	uint32_t          stage_pairs;
 	const float      *u8_to_unit;   /* [256]: (float)i / 255.0f, the byte→float division of texture.c:48-60 done once */
-	float             world_lo[3], world_inv[3];   /* top-level BVH bounds: lower corner and 1/extent (only used to BIN rays by origin cell, K4b) */
 };

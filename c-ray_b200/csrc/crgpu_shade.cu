@@ -5,7 +5,6 @@
  */
 #include "crgpu_wave.cuh"
 #include "crgpu_shade.cuh"
-#include <cstdlib>
 
 /* ---- K4: counting sort of the live rays by shading bucket --------------------------------------------------------------------
  * K2 left the bucket sizes in wb.hist[0..255].  Every block derives the same exclusive prefix, then ranks
@@ -13,24 +12,19 @@
  * with ONE global atomicAdd (cursor = wb.hist[256+k]).  Output: perm[bucket_base + rank] = live index.
  * Order inside a bucket is arbitrary; results do not depend on it (every path carries its own RNG + id). */
 #define CRG_BUCKET_ITEMS 8
-/* DIR = false: K4 (keys = hitKey, sizes hist[0..255], cursors hist[256..511], output perm).
- * DIR = true:  K4b, the same counting sort over the NEXT bounce's rays by direction bin (keys = dirKey written by K3, sizes
- *              hist[512..767], cursors hist[768..1023], output perm2): K2 hands rays to its lanes in perm2 order, so the 32 rays
- *              of a warp point into the same octant and walk the BVH in the same child order — fewer divergent steps. */
-template <bool DIR>
 __global__ void __launch_bounds__(256) k_bucket(WaveBuffers wb, int cur) {
 	__shared__ unsigned s_base[256], s_cnt[256], s_off[256];
 	const unsigned n = wb.counts[cur];
 	const unsigned t = threadIdx.x;
-	unsigned *__restrict__ sizes = wb.hist + (DIR ? 512 : 0);
-	unsigned *__restrict__ cursors = wb.hist + (DIR ? 768 : 256);
-	const unsigned char *__restrict__ keys = DIR ? wb.dirKey : wb.hitKey;
-	unsigned *__restrict__ out = DIR ? wb.perm2 : wb.perm;
+	unsigned *__restrict__ sizes = wb.hist;
+	unsigned *__restrict__ cursors = wb.hist + 256;
+	const unsigned char *__restrict__ keys = wb.hitKey;
+	unsigned *__restrict__ out = wb.perm;
 	s_cnt[t] = sizes[t];
 	__syncthreads();
 	if (t == 0u) { unsigned acc = 0u; for (int k = 0; k < 256; ++k) { s_base[k] = acc; acc += s_cnt[k]; } }
 	__syncthreads();
-	if (!DIR && blockIdx.x == 0u && t == 0u) wb.counts[4] = s_base[1];      /* = bucket 0's size: perm[0 .. counts[4]) are the misses (K3 split) */
+	if (blockIdx.x == 0u && t == 0u) wb.counts[4] = s_base[1];      /* = bucket 0's size: perm[0 .. counts[4]) are the misses (K3 split) */
 	const unsigned chunk = 256u * CRG_BUCKET_ITEMS;
 	for (unsigned c0 = blockIdx.x * chunk; c0 < n; c0 += gridDim.x * chunk) {
 		s_cnt[t] = 0u;
@@ -60,7 +54,6 @@ __global__ void __launch_bounds__(256) k_bucket(WaveBuffers wb, int cur) {
  * of the carried id remembers that L holds a value; a path that ends without any contribution writes zeros.  So K1
  * never has to clear L and most paths touch their L record exactly once. */
 #define CRG_ID_HAS_L 0x80000000u
-CRD void crg_prefetch_l2(const void *p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
 
 CRD void cr_add_radiance(float4 *__restrict__ Lbuf, unsigned &id, float r, float g, float b) {
 	const unsigned slot = id & ~CRG_ID_HAS_L;
@@ -106,28 +99,12 @@ CRD bool cr_shade_one(const DevScene &sc, float4 *__restrict__ Lbuf, v3 o, v3 d,
 	return false;
 }
 
-/* direction bin of a ray for K4b: sign octant (bvh.c:370-372 picks the near/far planes from exactly these bits), optionally
- * times the major axis.  Any binning is legal: the order rays are traced in never changes a result. */
-CRD unsigned cr_dir_bin(const DevScene &sc, v3 o, v3 d, int mode) {
-	unsigned key = (__float_as_uint(d.x) >> 31) | ((__float_as_uint(d.y) >> 31) << 1) | ((__float_as_uint(d.z) >> 31) << 2);
-	if (mode == 2) {
-		const float ax = fabsf(d.x), ay = fabsf(d.y), az = fabsf(d.z);
-		const unsigned major = (ax >= ay && ax >= az) ? 0u : (ay >= az ? 1u : 2u);
-		key |= major << 3;                       /* 0..23 */
-	} else if (mode == 3) {                      /* + origin cell in the world box: 4 x 2 x 4 cells -> 256 bins */
-		const float fx = (o.x - sc.world_lo[0]) * sc.world_inv[0], fy = (o.y - sc.world_lo[1]) * sc.world_inv[1], fz = (o.z - sc.world_lo[2]) * sc.world_inv[2];
-		const unsigned cx = (unsigned)fminf(fmaxf(fx * 4.0f, 0.0f), 3.0f), cy = (unsigned)fminf(fmaxf(fy * 2.0f, 0.0f), 1.0f), cz = (unsigned)fminf(fmaxf(fz * 4.0f, 0.0f), 3.0f);
-		key |= (cx << 3) | (cz << 5) | (cy << 7);
-	}
-	return key;
-}
-
 /* ---- K3 (+ compaction) ----------------------------------------------------------------------------------------------
- * PART 0: every ray of the queue.  PART 1 / 2: the two halves of a split launch — 1 = the misses (bucket 0 = perm[0 .. counts[4]):
- * background lookup + radiance, the path always ends, nothing to compact), 2 = the hits (perm[counts[4] .. n)).  The miss half
- * needs a third of the registers of the hit half, so it runs at twice the occupancy; on hdr.json 40% of all rays are misses. */
-template <int MINB, int PART, bool X>
-__global__ void __launch_bounds__(256, MINB) k_shade(const DevScene *__restrict__ scp, WaveBuffers wb, int cur, int depth, int maxDepth, int dirmode, int prefetch) {
+ * Two launches over the bucket order: PART 1 = the misses (bucket 0 = perm[0 .. counts[4]): background lookup + radiance, the
+ * path always ends, nothing to compact), 4 blocks per SM; PART 2 = the hits (perm[counts[4] .. n)), 3 blocks per SM.  The miss
+ * half needs a third of the registers of the hit half, so it runs at higher occupancy; on hdr.json 40% of all rays are misses. */
+template <int PART, bool X>
+__global__ void __launch_bounds__(256, PART == 1 ? 4 : 3) k_shade(const DevScene *__restrict__ scp, WaveBuffers wb, int cur, int depth, int maxDepth) {
 	const DevScene &sc = *scp;
 	const unsigned n = wb.counts[cur];
 	const int nxt = cur ^ 1;
@@ -145,32 +122,20 @@ __global__ void __launch_bounds__(256, MINB) k_shade(const DevScene *__restrict_
 		}
 		return;
 	}
-	__shared__ unsigned s_dir[256];                               /* direction-bin sizes of the rays this block writes (blockDim.x == 256) */
-	s_dir[threadIdx.x] = 0u;
-	__syncthreads();
 	if (blockIdx.x == 0 && threadIdx.x == 0) wb.counts[2] = 0u;   /* K2's work counter, for the next bounce */
 	if (blockIdx.x == 0) { wb.hist[threadIdx.x] = 0u; wb.hist[256 + threadIdx.x] = 0u; }   /* K2/K4 histogram + cursors (blockDim.x == 256) */
 	const unsigned lane = threadIdx.x & 31u;
 	/* whole warps iterate together so the ballot below is convergent */
-	const unsigned first = PART == 2 ? wb.counts[4] : 0u;
+	const unsigned first = wb.counts[4];
 	const unsigned nround = first + ((n - first + 31u) & ~31u);
-	/* perm is read two iterations ahead and the records it points to one iteration ahead (crg_prefetch_l2): the five 16-B gathers
-	 * through perm are the DRAM-latency loads of this loop (the scene itself is L2-resident), so they are L2 hits when needed */
-	unsigned j0 = first + blockIdx.x * blockDim.x + threadIdx.x;
-	unsigned i_cur = (prefetch && j0 < n) ? wb.perm[j0] : 0u, i_nxt = (prefetch && j0 + stride < n) ? wb.perm[j0 + stride] : 0u;
-	for (unsigned j = j0; j < nround; j += stride) {
-		const unsigned i_n2 = (prefetch && j + 2u * stride < n && j + 2u * stride > j) ? wb.perm[j + 2u * stride] : 0u;
+	for (unsigned j = first + blockIdx.x * blockDim.x + threadIdx.x; j < nround; j += stride) {
 		bool alive = false;
 		v3 p_next = v3make(0, 0, 0), d_next = v3make(0, 0, 0);
 		float wr = 0.f, wg = 0.f, wbl = 0.f;
 		unsigned id = 0u;
 		uint64_t rng = 0ull;
 		if (j < n) {
-			const unsigned i = prefetch ? i_cur : wb.perm[j];     /* bucket order: a warp shades one material */
-			if (prefetch && j + stride < n) {
-				crg_prefetch_l2(&wb.stA[cur][i_nxt]); crg_prefetch_l2(&wb.stB[cur][i_nxt]); crg_prefetch_l2(&wb.stC[cur][i_nxt]);
-				crg_prefetch_l2(&wb.hit[i_nxt]); crg_prefetch_l2(&wb.hitInst[i_nxt]);
-			}
+			const unsigned i = wb.perm[j];     /* bucket order: a warp shades one material */
 			const float4 a = wb.stA[cur][i];
 			const float4 b = wb.stB[cur][i];
 			const uint4 c = wb.stC[cur][i];
@@ -181,7 +146,7 @@ __global__ void __launch_bounds__(256, MINB) k_shade(const DevScene *__restrict_
 			wr = b.z; wg = b.w; wbl = __uint_as_float(c.x);
 			id = c.y;
 			rng = (uint64_t)c.z | ((uint64_t)c.w << 32);
-			alive = cr_shade_one<X, PART != 2>(sc, wb.L, v3make(a.x, a.y, a.z), v3make(a.w, b.x, b.y), hit, wr, wg, wbl, id, rng, depth, maxDepth, p_next, d_next);
+			alive = cr_shade_one<X, false>(sc, wb.L, v3make(a.x, a.y, a.z), v3make(a.w, b.x, b.y), hit, wr, wg, wbl, id, rng, depth, maxDepth, p_next, d_next);
 		}
 		/* order-preserving warp compaction, one atomic per warp */
 		const unsigned mask = __ballot_sync(0xffffffffu, alive);
@@ -194,18 +159,8 @@ __global__ void __launch_bounds__(256, MINB) k_shade(const DevScene *__restrict_
 				wb.stA[nxt][k] = make_float4(p_next.x, p_next.y, p_next.z, d_next.x);
 				wb.stB[nxt][k] = make_float4(d_next.y, d_next.z, wr, wg);
 				wb.stC[nxt][k] = make_uint4(__float_as_uint(wbl), id, (unsigned)(rng & 0xffffffffull), (unsigned)(rng >> 32));
-				if (dirmode) {
-					const unsigned key = cr_dir_bin(sc, p_next, d_next, dirmode);
-					wb.dirKey[k] = (unsigned char)key;
-					atomicAdd(&s_dir[key], 1u);
-				}
 			}
 		}
-		i_cur = i_nxt; i_nxt = i_n2;
-	}
-	if (dirmode) {
-		__syncthreads();
-		if (s_dir[threadIdx.x]) atomicAdd(&wb.hist[512 + threadIdx.x], s_dir[threadIdx.x]);
 	}
 }
 
@@ -328,7 +283,7 @@ __global__ void k_kat(const DevScene *__restrict__ scp, const int32_t *__restric
 }
 
 void crg_launch_bucket(const WaveBuffers &wb, int cur, int grid, cudaStream_t st) {
-	k_bucket<false><<<grid, 256, 0, st>>>(wb, cur);
+	k_bucket<<<grid, 256, 0, st>>>(wb, cur);
 }
 /* X (the last template argument): the scene contains node kinds only the complete interpreter knows (DevScene::has_xnodes, set at
  * upload) — every other scene runs the kernels in which that interpreter is not even linked */
@@ -336,36 +291,15 @@ void crg_launch_tail(const DevScene *dsc, const WaveBuffers &wb, int cur, int de
 	if (xnodes) k_tail<true><<<128, 128, 0, st>>>(dsc, wb, cur, depth, maxDepth);
 	else k_tail<false><<<128, 128, 0, st>>>(dsc, wb, cur, depth, maxDepth);
 }
-/* CRGPU_SHADE_MINB = 2|3|4 (blocks per SM of the hit/all kernel: 128 / 80 / 64 registers), CRGPU_SHADE_SPLIT = 0|1 (separate
- * miss kernel at 4 blocks per SM), CRGPU_SHADE_PREFETCH = 0|1 — read once; the defaults are what measured best (profiles/) */
-template <bool X>
-static void launch_shade(const DevScene *dsc, const WaveBuffers &wb, int cur, int depth, int maxDepth, int dirmode, int grid, cudaStream_t st) {
-	static const int minb = [] { const char *e = getenv("CRGPU_SHADE_MINB"); const int v = e ? atoi(e) : 3; return v >= 2 && v <= 4 ? v : 3; }();
-	static const int split = [] { const char *e = getenv("CRGPU_SHADE_SPLIT"); return e ? atoi(e) : 1; }();
-	static const int prefetch = [] { const char *e = getenv("CRGPU_SHADE_PREFETCH"); return e ? atoi(e) : 0; }();
-	if (split) {
-		k_shade<4, 1, X><<<grid, 256, 0, st>>>(dsc, wb, cur, depth, maxDepth, dirmode, prefetch);
-		if (minb == 3) k_shade<3, 2, X><<<grid, 256, 0, st>>>(dsc, wb, cur, depth, maxDepth, dirmode, prefetch);
-		else if (minb == 4) k_shade<4, 2, X><<<grid, 256, 0, st>>>(dsc, wb, cur, depth, maxDepth, dirmode, prefetch);
-		else k_shade<2, 2, X><<<grid, 256, 0, st>>>(dsc, wb, cur, depth, maxDepth, dirmode, prefetch);
-		return;
+void crg_launch_shade(const DevScene *dsc, const WaveBuffers &wb, int cur, int depth, int maxDepth, bool xnodes, int grid, cudaStream_t st) {
+	if (xnodes) {
+		k_shade<1, true><<<grid, 256, 0, st>>>(dsc, wb, cur, depth, maxDepth);
+		k_shade<2, true><<<grid, 256, 0, st>>>(dsc, wb, cur, depth, maxDepth);
+	} else {
+		k_shade<1, false><<<grid, 256, 0, st>>>(dsc, wb, cur, depth, maxDepth);
+		k_shade<2, false><<<grid, 256, 0, st>>>(dsc, wb, cur, depth, maxDepth);
 	}
-	if (minb == 3) k_shade<3, 0, X><<<grid, 256, 0, st>>>(dsc, wb, cur, depth, maxDepth, dirmode, prefetch);
-	else if (minb == 4) k_shade<4, 0, X><<<grid, 256, 0, st>>>(dsc, wb, cur, depth, maxDepth, dirmode, prefetch);
-	else k_shade<2, 0, X><<<grid, 256, 0, st>>>(dsc, wb, cur, depth, maxDepth, dirmode, prefetch);
 }
-void crg_launch_shade(const DevScene *dsc, const WaveBuffers &wb, int cur, int depth, int maxDepth, int dirmode, bool xnodes, int grid, cudaStream_t st) {
-	if (xnodes) launch_shade<true>(dsc, wb, cur, depth, maxDepth, dirmode, grid, st);
-	else launch_shade<false>(dsc, wb, cur, depth, maxDepth, dirmode, grid, st);
-}
-void crg_launch_dirsort(const WaveBuffers &wb, int nxt, int grid, cudaStream_t st) {
-	k_bucket<true><<<grid, 256, 0, st>>>(wb, nxt);
-}
-int crg_dir_mode(void) {
-	static const int mode = [] { const char *e = getenv("CRGPU_TRACE_SORT"); const int v = e ? atoi(e) : 0; return v >= 0 && v <= 3 ? v : 0; }();
-	return mode;
-}
-int crg_shade_launches_per_bounce(void) { const char *e = getenv("CRGPU_SHADE_SPLIT"); return (e ? atoi(e) : 1) ? 2 : 1; }
 void crg_launch_accumulate(float *fb, const float4 *L, const TileDesc &td, int W, int H, int grid, cudaStream_t st) {
 	k_accumulate<<<grid, 256, 0, st>>>(fb, L, td, W, H);
 }

@@ -6,7 +6,6 @@
 #include <mutex>
 #include "crgpu_wave.cuh"
 #include "crgpu_trace.cuh"
-#include <cstdlib>
 
 /* ---- pixel list of a tile set: blockIdx.y = tile, the block's threads walk its pixels row by row (crgpu_render_tiles) ---------------- */
 __global__ void __launch_bounds__(256) k_pixel_list(uint32_t *__restrict__ pixels, const int4 *__restrict__ rects, const unsigned *__restrict__ offs) {
@@ -42,7 +41,7 @@ __global__ void __launch_bounds__(256) k_generate(DevScene sc, WaveBuffers wb, T
 		wb.stC[0][id] = make_uint4(__float_as_uint(1.0f), id, (unsigned)(rng & 0xffffffffull), (unsigned)(rng >> 32));
 	}
 	if (blockIdx.x == 0 && threadIdx.x == 0) { wb.counts[0] = n; wb.counts[1] = 0u; wb.counts[2] = 0u; wb.counts[3] = 0u; }
-	if (blockIdx.x == 0) { for (int k = 0; k < 4; ++k) wb.hist[k * 256 + threadIdx.x] = 0u; }   /* blockDim.x == 256 */
+	if (blockIdx.x == 0) { for (int k = 0; k < 2; ++k) wb.hist[k * 256 + threadIdx.x] = 0u; }   /* blockDim.x == 256 */
 }
 
 /* ---- K2: persistent warps with dynamic ray refill ----------------------------------------------------------------------
@@ -53,54 +52,22 @@ __global__ void __launch_bounds__(256) k_generate(DevScene sc, WaveBuffers wb, T
  * out in lane order so neighbouring lanes still get neighbouring — coherent — rays). */
 #define CRG_REFILL 16
 #define CRG_NODE_BURST 3
-#define CRG_STAGE_MIN_RAYS 65536u
-#define CRG_DEFER_DEFAULT 0
+#define CRG_INST_MIN 8
 #define CRG_MAX_STEPS 8000000u   /* > 30x the node count of any scene that fits the 2^23-node address space we support */
 
-template <bool COUNT, int MINB, int DEFER>
-__global__ void __launch_bounds__(256, MINB) k_trace(DevScene sc, WaveBuffers wb, int cur, int refill, int burst, int sorted, int inst_min) {
+template <bool COUNT>
+__global__ void __launch_bounds__(256, 3) k_trace(DevScene sc, WaveBuffers wb, int cur) {
 	const unsigned n = wb.counts[cur];
 	const unsigned lane = threadIdx.x & 31u;
 	const float4 *__restrict__ stA = wb.stA[cur];
 	const float4 *__restrict__ stB = wb.stB[cur];
 	TraceCounters tc = { 0u, 0u, 0u, 0u };
 	__shared__ unsigned s_hist[256];
-	__shared__ CoopScratch s_coop[DEFER == 2 ? 8 : 1];   /* one per warp (blockDim.x == 256) */
 	s_hist[threadIdx.x] = 0u;            /* blockDim.x == 256 */
-	/* K3 + K4b of the previous bounce are done with the direction-bin counters: clear them for this bounce's K3 */
-	if (blockIdx.x == 0) { wb.hist[512 + threadIdx.x] = 0u; wb.hist[768 + threadIdx.x] = 0u; }
-	const unsigned *__restrict__ order = sorted ? wb.perm2 : nullptr;     /* rays in direction-bin order (see k_dirsort) */
 	__syncthreads();
-	/* ---- stage the top-of-tree pair nodes into shared memory: one TMA bulk copy (cp.async.bulk, SASS UBLKCP) per
-	 *      block, completion signalled on an mbarrier; skipped for the small tail launches where it cannot pay off */
-	extern __shared__ __align__(128) unsigned char s_dyn[];
-	__shared__ __align__(8) unsigned long long s_mbar;
-	const PairNode *snodes = nullptr;
-	if (sc.stage_pairs && n >= CRG_STAGE_MIN_RAYS) {
-		const unsigned bytes = sc.stage_pairs * (unsigned)sizeof(PairNode);
-		const unsigned mbar = (unsigned)__cvta_generic_to_shared(&s_mbar);
-		const unsigned dst = (unsigned)__cvta_generic_to_shared(s_dyn);
-		if (threadIdx.x == 0) {
-			asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(mbar));
-			asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-		}
-		__syncthreads();
-		if (threadIdx.x == 0) {
-			asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(mbar), "r"(bytes) : "memory");
-			asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-						 ::"r"(dst), "l"(sc.stage_img), "r"(bytes), "r"(mbar) : "memory");
-		}
-		unsigned ok = 0u;
-		while (!ok) {
-			asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], 0;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-						 : "=r"(ok) : "r"(mbar) : "memory");
-		}
-		snodes = reinterpret_cast<const PairNode *>(s_dyn);
-	}
 	uint32_t stack[2 * CRG_MAX_STACK + 2];
 	Traversal<COUNT> tr;
 	tr.stack = stack;
-	tr.snodes = snodes;
 	tr.begin(sc, v3make(0.f, 0.f, 0.f), v3make(0.f, 0.f, 1.f));   /* every lane holds a VALID (idle) state from the start */
 	bool busy = false;
 	bool exhausted = false;          /* warp-uniform: the work counter ran past n */
@@ -108,7 +75,7 @@ __global__ void __launch_bounds__(256, MINB) k_trace(DevScene sc, WaveBuffers wb
 	unsigned steps = 0u;             /* safety net: a lane that exceeds CRG_MAX_STEPS is abandoned and flagged */
 	while (true) {
 		unsigned active = __ballot_sync(0xffffffffu, busy);
-		if (!exhausted && __popc(active) < refill) {
+		if (!exhausted && __popc(active) < CRG_REFILL) {
 			const unsigned idle = ~active;
 			const unsigned nidle = (unsigned)__popc(idle);
 			unsigned base = 0u;
@@ -117,10 +84,9 @@ __global__ void __launch_bounds__(256, MINB) k_trace(DevScene sc, WaveBuffers wb
 			if (base + nidle >= n) exhausted = true;
 			const unsigned slot = base + (unsigned)__popc(idle & ((1u << lane) - 1u));
 			if (!busy && slot < n) {
-				const unsigned i = order ? order[slot] : slot;
-				const float4 a = stA[i];
-				const float4 b = stB[i];
-				ray = i;
+				const float4 a = stA[slot];
+				const float4 b = stB[slot];
+				ray = slot;
 				steps = 0u;
 				tr.begin(sc, v3make(a.x, a.y, a.z), v3make(a.w, b.x, b.y));
 				busy = true;
@@ -132,23 +98,20 @@ __global__ void __launch_bounds__(256, MINB) k_trace(DevScene sc, WaveBuffers wb
 		 * top-level leaf (instance work) or finish wait here, so that the instance / write-back code below runs
 		 * for many lanes at once instead of being serialised against node steps in every iteration. */
 #pragma unroll 1
-		for (int k = 0; k < burst; ++k) {
+		for (int k = 0; k < CRG_NODE_BURST; ++k) {
 			const bool wn = busy && tr.wants_node();
 			if (!__any_sync(0xffffffffu, wn)) break;
-			if (wn) { tr.template node_step<DEFER != 0>(sc, &tc); ++steps; }
+			if (wn) { tr.node_step(sc, &tc); ++steps; }
 		}
-		/* Phase T (DEFER): the triangles of every lane that reached a leaf during the burst, together */
-		if (DEFER == 2) cr_coop_leaves<COUNT>(tr, busy && tr.wants_leaf(), sc, s_coop[threadIdx.x >> 5], lane, &tc);   /* dealt over the warp */
-		else if (DEFER == 1 && busy && tr.wants_leaf()) tr.leaf_step(sc, &tc);
 		/* Phase I: one pending instance (ray transform + sphere test, or entry into a mesh BVH).  ncu (profiles/r01: 19.8% of K2's
 		 * warp instructions ran with fewer than 2 active lanes, almost all of them here): lanes reach a top-level leaf at different
 		 * iterations, so running this ~100-instruction block whenever ANY lane wants it means running it for one lane.  Lanes
-		 * therefore WAIT here until at least `inst_min` of them want an instance step, or no lane of the warp can take a node step. */
+		 * therefore WAIT here until at least CRG_INST_MIN of them want an instance step, or no lane of the warp can take a node step. */
 		{
 			const bool wi = busy && tr.wants_instance();
 			const unsigned mi = __ballot_sync(0xffffffffu, wi);
 			if (mi) {
-				bool go = (int)__popc(mi) >= inst_min;
+				bool go = __popc(mi) >= CRG_INST_MIN;
 				if (!go) go = !__any_sync(0xffffffffu, busy && tr.wants_node());
 				if (go && wi) { tr.instance_step(sc, &tc); ++steps; }
 			}
@@ -194,60 +157,35 @@ __global__ void __launch_bounds__(256, MINB) k_trace(DevScene sc, WaveBuffers wb
 void crg_launch_generate(const DevScene &sc, const WaveBuffers &wb, const TileDesc &td, int grid, cudaStream_t st) {
 	k_generate<<<grid, 256, 0, st>>>(sc, wb, td);
 }
-/* K2 is persistent: the grid is exactly the number of blocks the device can keep resident.  MINB (blocks per SM
- * the compiler must make room for: 2 -> <=128 registers, 3 -> <=80, 4 -> <=64) trades registers for latency-hiding warps;
- * CRGPU_TRACE_MINB=2|3 overrides the default for experiments. */
+/* K2 is persistent: the grid is exactly the number of blocks the device can keep resident (3 per SM: the launch bounds
+ * leave the compiler 80 registers per thread). */
 #ifndef CRG_MAX_DEVICES
 #define CRG_MAX_DEVICES 64
 #endif
-template <bool COUNT, int MINB, int DEFER>
-static void launch_trace_variant(const DevScene &sc, const WaveBuffers &wb, int cur, bool sorted, cudaStream_t st) {
-	/* launch shape per DEVICE: the host mirror drives several GPUs from one process (one thread each), and both the
-	 * occupancy answer and the opt-in shared-memory attribute belong to a device, not to the process */
-	struct Shape { int grid; size_t smem; };
-	static Shape shapes[CRG_MAX_DEVICES];
-	static std::mutex shapes_lock;
-	const size_t smem = (size_t)sc.stage_pairs * sizeof(PairNode);
+template <bool COUNT>
+static void launch_trace_variant(const DevScene &sc, const WaveBuffers &wb, int cur, cudaStream_t st) {
+	/* grid per DEVICE: the host mirror drives several GPUs from one process (one thread each), and the occupancy answer
+	 * belongs to a device, not to the process */
+	static int grids[CRG_MAX_DEVICES];
+	static std::mutex grids_lock;
 	int dev = 0;
 	cudaGetDevice(&dev);
 	int grid;
 	{
-		std::lock_guard<std::mutex> guard(shapes_lock);
-		Shape &sh = shapes[dev >= 0 && dev < CRG_MAX_DEVICES ? dev : 0];
-		if (!sh.grid || sh.smem != smem) {
+		std::lock_guard<std::mutex> guard(grids_lock);
+		int &g = grids[dev >= 0 && dev < CRG_MAX_DEVICES ? dev : 0];
+		if (!g) {
 			int sms = 0, occ = 0;
 			cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-			cudaFuncSetAttribute(k_trace<COUNT, MINB, DEFER>, cudaFuncAttributeMaxDynamicSharedMemorySize, CRG_STAGE_PAIRS * (int)sizeof(PairNode));
-			cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_trace<COUNT, MINB, DEFER>, 256, smem);
-			sh.grid = sms * (occ > 0 ? occ : 1);
-			sh.smem = smem;
+			cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_trace<COUNT>, 256, 0);
+			g = sms * (occ > 0 ? occ : 1);
 		}
-		grid = sh.grid;
+		grid = g;
 	}
-	static const int refill = [] { const char *e = getenv("CRGPU_TRACE_REFILL"); const int v = e ? atoi(e) : CRG_REFILL; return v >= 1 && v <= 32 ? v : CRG_REFILL; }();
-	static const int burst = [] { const char *e = getenv("CRGPU_TRACE_BURST"); const int v = e ? atoi(e) : (DEFER ? 4 : CRG_NODE_BURST); return v >= 1 ? v : CRG_NODE_BURST; }();
-	static const int inst_min = [] { const char *e = getenv("CRGPU_TRACE_INSTMIN"); const int v = e ? atoi(e) : 8; return v >= 1 && v <= 32 ? v : 8; }();
-	k_trace<COUNT, MINB, DEFER><<<grid, 256, smem, st>>>(sc, wb, cur, refill, burst, sorted ? 1 : 0, inst_min);
+	k_trace<COUNT><<<grid, 256, 0, st>>>(sc, wb, cur);
 }
 
-void crg_launch_trace(const DevScene &sc, const WaveBuffers &wb, int cur, bool count, bool sorted, int grid, cudaStream_t st) {
-	(void)grid;
-	static const int minb = [] { const char *e = getenv("CRGPU_TRACE_MINB"); const int v = e ? atoi(e) : 3; return v >= 2 && v <= 4 ? v : 3; }();
-	/* CRGPU_TRACE_DEFER: 0 = triangles tested inside the node step, 1 = lanes wait and test their own leaf after the burst,
-	 * 2 = lanes wait and the warp deals the (ray, triangle) pairs over its 32 lanes (cr_coop_leaves) */
-	static const int defer = [] { const char *e = getenv("CRGPU_TRACE_DEFER"); const int v = e ? atoi(e) : CRG_DEFER_DEFAULT; return v >= 0 && v <= 2 ? v : CRG_DEFER_DEFAULT; }();
-	if (count) {
-		if (defer == 2) launch_trace_variant<true, 3, 2>(sc, wb, cur, sorted, st);
-		else if (defer == 1) launch_trace_variant<true, 3, 1>(sc, wb, cur, sorted, st);
-		else launch_trace_variant<true, 3, 0>(sc, wb, cur, sorted, st);
-		return;
-	}
-#define CRG_TRACE_DISPATCH(D) do { \
-		if (minb == 4) launch_trace_variant<false, 4, D>(sc, wb, cur, sorted, st); \
-		else if (minb == 2) launch_trace_variant<false, 2, D>(sc, wb, cur, sorted, st); \
-		else launch_trace_variant<false, 3, D>(sc, wb, cur, sorted, st); } while (0)
-	if (defer == 2) CRG_TRACE_DISPATCH(2);
-	else if (defer == 1) CRG_TRACE_DISPATCH(1);
-	else CRG_TRACE_DISPATCH(0);
-#undef CRG_TRACE_DISPATCH
+void crg_launch_trace(const DevScene &sc, const WaveBuffers &wb, int cur, bool count, cudaStream_t st) {
+	if (count) launch_trace_variant<true>(sc, wb, cur, st);
+	else launch_trace_variant<false>(sc, wb, cur, st);
 }

@@ -82,13 +82,8 @@ CRD RaySetup cr_ray_setup(v3 o, v3 d) {                                         
  * -march=native build) and a*b+c otherwise (the strict oracle build).  The slab test only decides which nodes
  * are ENTERED, never a hit distance, and both variants are conservative; the survey measured bit-identical
  * framebuffers between them on hdr.json and venus.json, and tests/test_gpu_parity.py holds the fused variant to
- * exact hit records against the un-fused oracle.  Fused = 6 FFMA per child instead of 6 FMUL + 6 FADD.
- * Build with -DCRG_SLAB_UNFUSED to get the two-rounding form. */
-#ifdef CRG_SLAB_UNFUSED
-#define CR_SLAB_MAD(a, b, c) ((a) * (b) + (c))
-#else
+ * exact hit records against the un-fused oracle.  Fused = 6 FFMA per child instead of 6 FMUL + 6 FADD. */
 #define CR_SLAB_MAD(a, b, c) __fmaf_rn((a), (b), (c))
-#endif
 
 /* Slab test of one child.  For ordinary rays this is intersectNode verbatim (bvh.c:326-352).
  *
@@ -227,30 +222,25 @@ struct Traversal {
 	v3 o, d;               /* ray of the current level */
 	RaySetup rs;
 	const PairNode *__restrict__ base;
-	const PairNode *snodes;        /* shared-memory copy of DevScene.stage_img (NULL: not staged) */
-	uint32_t stageBase, stageCount;/* nodes [0, stageCount) of the current BVH live at snodes[stageBase + node] */
 	const PackedTri *__restrict__ tris;
 	uint32_t slotBase, node, topNext;
 	uint32_t pendA, cntA, pendB, cntB;     /* pending top-level leaf items: A (left leaf) before B (right leaf) */
-	uint32_t leafA, leafB, leafN;          /* DEFER: bottom-level leaf triangles not yet tested — slots [leafA, +nA) then [leafB, +nB), leafN = nA | nB << 16 */
 	int sp, spBase, curInst;
 	bool bottom, instHit;
 	uint32_t *stack;       /* 2*CRG_MAX_STACK+2 entries of thread-local memory, owned by the caller (keeps the scalars in registers) */
 
-	CRD bool done() const { return !bottom && (cntA | cntB) == 0u && node == CRG_END && leafN == 0u; }
+	CRD bool done() const { return !bottom && (cntA | cntB) == 0u && node == CRG_END; }
 
 	CRD void begin(const DevScene &sc, v3 ro, v3 rd) {
 		best.t = CR_FLT_MAX; best.u = 0.0f; best.v = 0.0f; best.inst = -1; best.prim = 0u;
 		wo = ro; wd = rd; o = ro; d = rd;
 		rs = cr_ray_setup(o, d);
 		base = sc.pairs + sc.top.pair_offset;
-		stageBase = sc.top.stage_base; stageCount = snodes ? sc.top.stage_count : 0u;
 		tris = sc.tris;
 		slotBase = 0u; node = 0u; topNext = CRG_END;
 		pendA = 0u; cntA = 0u; pendB = 0u; cntB = 0u;
 		sp = 0; spBase = 0; curInst = -1;
 		bottom = false; instHit = false;
-		leafA = 0u; leafB = 0u; leafN = 0u;
 		if (sc.top.node_count < 1) {                                               /* bvh.c:362-365 */
 			node = CRG_END;
 		} else if (sc.top.node_count == 1) {                                       /* bvh.c:382-387 */
@@ -260,8 +250,7 @@ struct Traversal {
 		}
 	}
 
-	CRD bool wants_node() const { return leafN == 0u && (bottom || ((cntA | cntB) == 0u && node != CRG_END)); }
-	CRD bool wants_leaf() const { return leafN != 0u; }
+	CRD bool wants_node() const { return bottom || ((cntA | cntB) == 0u && node != CRG_END); }
 	CRD bool wants_instance() const { return !bottom && (cntA | cntB) != 0u; }
 
 	/* one iteration of the flat loop; precondition: !done() */
@@ -278,38 +267,18 @@ struct Traversal {
 			o = wo; d = wd;
 			rs = cr_ray_setup(o, d);
 			base = sc.pairs + sc.top.pair_offset;
-			stageBase = sc.top.stage_base; stageCount = snodes ? sc.top.stage_count : 0u;
 			node = topNext;
 			spBase = 0;
 		}
 	}
 
-	/* DEFER: the triangles of the leaf/leaves the last node step reached (left leaf, then right leaf: bvh.c:402-418).  Until this has
-	 * run the lane takes no further node step, so the visiting order and the distance every later box is culled with are exactly
-	 * those of the in-line version; only the warp's interleaving differs: lanes that reached a leaf WAIT, and all waiting lanes of
-	 * the warp test their triangles together after the node burst (profiles/: K2 warp model, policy "leaves wait"). */
-	CRD void leaf_step(const DevScene &sc, TraceCounters *ctr) {
-		instHit |= cr_leaf_tris2<COUNT>(tris, slotBase, leafA, leafN & 0xffffu, leafB, leafN >> 16, o, d, best, ctr);
-		leafN = 0u;
-		finish_bottom(sc);
-	}
-
-	/* precondition: wants_node().  DEFER = true: leaf triangles are left pending for leaf_step() */
-	template <bool DEFER = false>
+	/* precondition: wants_node() */
 	CRD void node_step(const DevScene &sc, TraceCounters *ctr) {
 		{
 			/* ---- one child-pair step (bvh.c:391-439) */
-			float4 q0, q1, q2;
-			uint4 q3;
-			if (node < stageCount) {                     /* top of the tree: staged in shared memory by TMA */
-				const float4 *p4 = reinterpret_cast<const float4 *>(snodes + stageBase + node);
-				q0 = p4[0]; q1 = p4[1]; q2 = p4[2];
-				q3 = *reinterpret_cast<const uint4 *>(p4 + 3);
-			} else {
-				const float4 *p4 = reinterpret_cast<const float4 *>(base + node);
-				q0 = __ldg(p4 + 0); q1 = __ldg(p4 + 1); q2 = __ldg(p4 + 2);
-				q3 = __ldg(reinterpret_cast<const uint4 *>(p4 + 3));
-			}
+			const float4 *p4 = reinterpret_cast<const float4 *>(base + node);
+			const float4 q0 = __ldg(p4 + 0), q1 = __ldg(p4 + 1), q2 = __ldg(p4 + 2);
+			const uint4 q3 = __ldg(reinterpret_cast<const uint4 *>(p4 + 3));
 			const float lb[6] = { q0.x, q0.y, q0.z, q0.w, q1.x, q1.y };
 			const float rb[6] = { q1.z, q1.w, q2.x, q2.y, q2.z, q2.w };
 			if (COUNT) ctr->pairs++;
@@ -334,12 +303,8 @@ struct Traversal {
 				const uint32_t nL = (hitL && leafL) ? (q3.z & ~CRG_LEAF_BIT) : 0u;
 				const uint32_t nR = (hitR && leafR) ? (q3.w & ~CRG_LEAF_BIT) : 0u;
 				node = next;
-				if (DEFER && (nL + nR) != 0u && nL < 65536u && nR < 65536u) {
-					leafA = q3.x; leafB = q3.y; leafN = nL | (nR << 16);               /* tested by leaf_step(), then finish_bottom() */
-				} else {
-					if (nL + nR) instHit |= cr_leaf_tris2<COUNT>(tris, slotBase, q3.x, nL, q3.y, nR, o, d, best, ctr);
-					finish_bottom(sc);
-				}
+				if (nL + nR) instHit |= cr_leaf_tris2<COUNT>(tris, slotBase, q3.x, nL, q3.y, nR, o, d, best, ctr);
+				finish_bottom(sc);
 			} else {
 				if (hitL && leafL) { pendA = q3.x; cntA = q3.z & ~CRG_LEAF_BIT; }
 				if (hitR && leafR) { pendB = q3.y; cntB = q3.w & ~CRG_LEAF_BIT; }
@@ -382,7 +347,6 @@ struct Traversal {
 					o = oo; d = od;
 					rs = cr_ray_setup(o, d);
 					base = sc.pairs + __ldg(&bvh->pair_offset);
-					stageBase = __ldg(&bvh->stage_base); stageCount = snodes ? __ldg(&bvh->stage_count) : 0u;
 					tris = sc.tris + slotOff;
 					slotBase = slotOff;
 					curInst = cur;
@@ -398,87 +362,11 @@ struct Traversal {
 	}
 };
 
-/* ---- cooperative leaf phase (K2, DEFER == 2) ------------------------------------------------------------------------------------
- * ncu (profiles/r02): a quarter of K2's warp instructions are Möller–Trumbore tests executed with ~2 active lanes — at any step only
- * one or two lanes of a warp stand at a leaf, and the warp then runs the per-lane triangle loop max(leaf size) times for them.
- * Here the lanes that reached a leaf WAIT (Traversal::leafN, as in DEFER == 1) and, after the node burst, the warp deals all their
- * (ray, triangle) pairs out over its 32 lanes: one pass of the triangle code tests up to 32 pairs of up to 32 different rays.
- * The ray of a pair is read from its owner lane with shuffles; candidates go back through 3 x 32 floats of shared memory per warp and
- * every owner takes its winner IN LEAF ORDER with the reference's strict `t < distance` (poly.c:48, bvh.c:455-459: the first of equal
- * distances wins), so hit records stay bit-identical.  Must be called by all 32 lanes of the warp (convergent). */
-struct CoopScratch { float t[32], u[32], v[32]; unsigned owner[32]; };
-
-template <bool COUNT>
-CRD void cr_coop_leaves(Traversal<COUNT> &tr, bool has, const DevScene &sc, CoopScratch &cs, unsigned lane, TraceCounters *ctr) {
-	const unsigned FULL = 0xffffffffu;
-	unsigned pending = __ballot_sync(FULL, has);
-	while (pending) {
-		const unsigned nA = tr.leafN & 0xffffu, nB = tr.leafN >> 16;
-		unsigned cnt = has ? nA + nB : 0u;
-		if (cnt > 32u) { tr.leaf_step(sc, ctr); has = false; cnt = 0u; }      /* an oversized leaf pair: the lane's own loop (rare) */
-		unsigned incl = cnt;
-#pragma unroll
-		for (unsigned dlt = 1u; dlt < 32u; dlt <<= 1) { const unsigned x = __shfl_up_sync(FULL, incl, dlt); if (lane >= dlt) incl += x; }
-		const bool fits = has && incl <= 32u;                 /* incl is non-decreasing over lanes: the lanes that fit form a prefix */
-		const unsigned excl = incl - cnt;
-		const unsigned startMask = __reduce_or_sync(FULL, fits ? (1u << (excl & 31u)) : 0u);
-		const unsigned tot = __reduce_max_sync(FULL, fits ? incl : 0u);
-		if (fits) cs.owner[excl & 31u] = lane;
-		__syncwarp();
-		/* pair `lane` of this round: owner = the lane whose segment [excl, incl) holds it */
-		unsigned seg = 0u, ow = lane;
-		if (lane < tot) { seg = 31u - (unsigned)__clz((int)(startMask & (0xffffffffu >> (31u - lane)))); ow = cs.owner[seg]; }
-		const float ox = __shfl_sync(FULL, tr.o.x, ow), oy = __shfl_sync(FULL, tr.o.y, ow), oz = __shfl_sync(FULL, tr.o.z, ow);
-		const float dx = __shfl_sync(FULL, tr.d.x, ow), dy = __shfl_sync(FULL, tr.d.y, ow), dz = __shfl_sync(FULL, tr.d.z, ow);
-		const unsigned lA = __shfl_sync(FULL, tr.leafA, ow), lB = __shfl_sync(FULL, tr.leafB, ow), lN = __shfl_sync(FULL, tr.leafN, ow);
-		const unsigned sb = __shfl_sync(FULL, tr.slotBase, ow);
-		if (lane < tot) {
-			const unsigned k = lane - seg, onA = lN & 0xffffu;
-			const unsigned slot = k < onA ? lA + k : lB + (k - onA);
-			const float4 *t4 = reinterpret_cast<const float4 *>(sc.tris + sb + slot);
-			const float4 a = __ldg(t4 + 0), b = __ldg(t4 + 1), c4 = __ldg(t4 + 2);
-			if (COUNT) ctr->tris++;
-			const v3 o = v3make(ox, oy, oz), d = v3make(dx, dy, dz);
-			const v3 v0 = v3make(a.x, a.y, a.z), e1 = v3make(a.w, b.x, b.y), e2 = v3make(b.z, b.w, c4.x);
-			const v3 n = v3make(c4.y, c4.z, c4.w);
-			const v3 c = v3sub(v0, o);
-			const v3 r = v3cross(d, c);
-			const float invDet = cr_div(1.0f, v3dot(n, d));
-			const float u = v3dot(r, e2) * invDet;
-			const float v = v3dot(r, e1) * invDet;
-			float tt = __int_as_float(0x7f800000);              /* +inf: never `< distance` */
-			if (u >= 0.0f && v >= 0.0f && u + v <= 1.0f) {
-				const float t = v3dot(n, c) * invDet;
-				if (t >= 0.0f) tt = t;
-			}
-			cs.t[lane] = tt; cs.u[lane] = u; cs.v[lane] = v;
-		}
-		__syncwarp();
-		if (fits) {
-			float bt = tr.best.t;
-			int kb = -1;
-			for (unsigned k = 0u; k < cnt; ++k) { const float x = cs.t[excl + k]; if (x < bt) { bt = x; kb = (int)k; } }
-			if (kb >= 0) {
-				const unsigned k = (unsigned)kb;
-				tr.best.t = bt; tr.best.u = cs.u[excl + k]; tr.best.v = cs.v[excl + k];
-				tr.best.prim = tr.slotBase + (k < nA ? tr.leafA + k : tr.leafB + (k - nA));
-				tr.instHit = true;
-			}
-			tr.leafN = 0u;
-			tr.finish_bottom(sc);
-			has = false;
-		}
-		__syncwarp();
-		pending = __ballot_sync(FULL, has);
-	}
-}
-
 template <bool COUNT>
 CRD Hit cr_closest_hit(const DevScene &sc, v3 wo, v3 wd, TraceCounters *ctr) {
 	uint32_t stack[2 * CRG_MAX_STACK + 2];
 	Traversal<COUNT> tr;
 	tr.stack = stack;
-	tr.snodes = nullptr;
 	tr.begin(sc, wo, wd);
 	while (!tr.done()) tr.step(sc, ctr);
 	return tr.best;

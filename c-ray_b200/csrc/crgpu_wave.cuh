@@ -35,10 +35,7 @@ struct WaveBuffers {
 	float4 *L;
 	unsigned char *hitKey;  /* shading bucket of the hit: 0 = miss, else min(material+1, 255) */
 	unsigned *perm;         /* K4 output: live indices grouped by bucket */
-	unsigned char *dirKey;  /* direction bin of every ray K3 wrote for the next bounce (octant [+ major axis]) */
-	unsigned *perm2;        /* K4b output: the next bounce's rays grouped by direction bin — the order K2 hands them to its lanes */
-	unsigned *hist;         /* [256] bucket sizes (filled by K2), [256..511] K4 cursors, [512..767] direction-bin sizes (filled by K3),
-	                           [768..1023] K4b cursors */
+	unsigned *hist;         /* [256] bucket sizes (filled by K2), [256..511] K4 cursors */
 	unsigned *counts;       /* [0],[1]: live counts of the ping-pong halves; [2]: K2's work counter (next ray to hand out); [3]: tail-kernel block counter; [4]: number of misses of this bounce (K4 -> K3 split) */
 	unsigned long long *stats; /* [0] rays, [1] pairs, [2] tris, [3] spheres, [4] insts */
 };
@@ -58,13 +55,10 @@ __device__ __forceinline__ void crg_pixel_xy(const TileDesc &td, unsigned px, in
 /* launchers (defined in crgpu_trace.cu / crgpu_shade.cu); `dsc` is the device copy of `sc` */
 void crg_launch_pixel_list(uint32_t *pixels, const int4 *rects, const unsigned *offs, int nrects, cudaStream_t st);
 void crg_launch_generate(const DevScene &sc, const WaveBuffers &wb, const TileDesc &td, int grid, cudaStream_t st);
-void crg_launch_trace(const DevScene &sc, const WaveBuffers &wb, int cur, bool count, bool sorted, int grid, cudaStream_t st);
-void crg_launch_dirsort(const WaveBuffers &wb, int nxt, int grid, cudaStream_t st);
-int crg_dir_mode(void);   /* 0 = off, 1 = octant (8 bins), 2 = octant x major axis (24 bins), 3 = octant x origin cell (256 bins) */
+void crg_launch_trace(const DevScene &sc, const WaveBuffers &wb, int cur, bool count, cudaStream_t st);
 void crg_launch_bucket(const WaveBuffers &wb, int cur, int grid, cudaStream_t st);
 void crg_launch_tail(const DevScene *dsc, const WaveBuffers &wb, int cur, int depth, int maxDepth, bool xnodes, cudaStream_t st);
-void crg_launch_shade(const DevScene *dsc, const WaveBuffers &wb, int cur, int depth, int maxDepth, int dirmode, bool xnodes, int grid, cudaStream_t st);
-int crg_shade_launches_per_bounce(void);
+void crg_launch_shade(const DevScene *dsc, const WaveBuffers &wb, int cur, int depth, int maxDepth, bool xnodes, int grid, cudaStream_t st);
 void crg_launch_accumulate(float *fb, const float4 *L, const TileDesc &td, int W, int H, int grid, cudaStream_t st);
 void crg_launch_to_srgb8(const float *fb, uint8_t *out, size_t n, int grid, cudaStream_t st);
 void crg_launch_kat(const DevScene *dsc, const int32_t *xyp, int count, void *out, cudaStream_t st);
